@@ -172,26 +172,6 @@ def test_graph_host_and_device_paths_agree():
         e.close()
 
 
-def test_partition_invariance():
-    """One slab of 2N envs == two slabs of N envs with global env indices (SURVEY 8e / Appendix F.5): bitwise."""
-    import torch
-    from gym_xarm_b200 import XarmVecEnv
-    n = 128
-    whole = XarmVecEnv("pick_and_place", 2 * n, device="cuda:0", seed=9)
-    parts = [XarmVecEnv("pick_and_place", n, device="cuda:0", seed=9, env_index_base=k * n) for k in range(2)]
-    whole.reset()
-    for p in parts:
-        p.reset()
-    rng = np.random.default_rng(1)
-    for t in range(55):
-        a = torch.from_numpy(rng.uniform(-1, 1, (2 * n, 4)).astype(np.float32)).cuda()
-        ow, rw, dw, _ = whole.step(a)
-        for k, p in enumerate(parts):
-            op, rp, dp, _ = p.step(a[k * n:(k + 1) * n].contiguous())
-            assert torch.equal(ow["observation"][k * n:(k + 1) * n], op["observation"])
-            assert torch.equal(rw[k * n:(k + 1) * n], rp) and torch.equal(dw[k * n:(k + 1) * n], dp)
-
-
 def test_full_size_properties():
     """BASELINE size (131072 PickAndPlace envs): size-independent invariants over 60 auto-resetting steps."""
     import torch
